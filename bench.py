@@ -28,6 +28,8 @@ algorithmic GB/s against the measured HBM peak.  Workload = BASELINE config 2 ("
             every rank renders its interleaved 8-row bands of all frames with one launch and the copy
             engines scatter them into the frames on rank 0 (2-D peer copies); the reassembled frames are
             compared with a single-GPU render (`config.reassembly_identical_to_single_gpu`).
+  --dump-outputs DIR   the RGBA8 frames of the last timed step (and of the last e2e step) as float32 .npy files, the
+            same fixed sample of pixels on every run, so that two builds can be compared output for output.
 
 Kernels: batches (the `value` / `e2e` legs) run the inline-shading kernel, single-view launches (the `cli` leg,
 launch_renderer) the shading-queue kernel; `config.kernel_variant` names the batch kernel (DESIGN.md 4).
@@ -43,6 +45,7 @@ import os
 import re
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -55,6 +58,33 @@ W = H = 800
 N_POSES = 200
 WORKLOAD_SYNTH = ("synthetic lego-like SH16 N3Tree stand-in (depth 10, seed 0; real lego tree.npz is an external "
                   "download), 800x800, 200 NeRF-synthetic test-orbit poses, default RenderOptions")
+DUMP_PIXELS = 1 << 20          # --dump-outputs: at most 1 Mi RGBA pixels (16 MB as float32) per array
+_TMP = None
+
+
+def tmp_dir() -> str:
+    """This run's scratch directory (tree.npz and pose files for the CLI and reference legs), removed at exit."""
+    global _TMP
+    if _TMP is None:
+        _TMP = tempfile.TemporaryDirectory(prefix="vr_bench_")
+    return _TMP.name
+
+
+def frame_sample(frames) -> np.ndarray:
+    """float32 [n, 4] copy of an RGBA8 frame stack [V, H, W, 4] (CUDA or host tensor): every pixel when there are at
+    most DUMP_PIXELS, else the same DUMP_PIXELS pixels on every run (seed 0, in index order)."""
+    import torch
+    px = frames.reshape(-1, 4)
+    if px.shape[0] > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(px.shape[0], DUMP_PIXELS, replace=False))
+        px = px[torch.from_numpy(idx).to(px.device)]
+    return px.float().cpu().numpy()
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def env_int(name, default):
@@ -205,7 +235,7 @@ class Scene:
     def npz_path(self) -> str:
         if self.real_npz:
             return self.real_npz
-        path = "/tmp/vr_bench_tree.npz"
+        path = os.path.join(tmp_dir(), "vr_bench_tree.npz")
         if not os.path.exists(path):
             self.st.save_npz(path)
         return path
@@ -261,7 +291,7 @@ def cli_leg(scene: Scene, exe: str, n_frames: int = N_POSES):
         return None
     try:
         npz = scene.npz_path()
-        pdir = "/tmp/vr_bench_poses"
+        pdir = os.path.join(tmp_dir(), "vr_bench_poses")
         ppaths = synth.write_pose_files(scene.poses[:n_frames], pdir, synth.focal_for(W))
         cmd = [exe, npz, "-w", str(W), "-h", str(H), "--fx", str(synth.focal_for(W))] + ppaths
         best = None
@@ -408,9 +438,8 @@ def reference_config4(args):
         line["unavailable"] = "oracle/_ref not built or no GPU"
         return line
     st, poses = config4_scene()
-    path = "/tmp/vr_config4_tree.npz"
-    if not os.path.exists(path):
-        st.save_npz(path)
+    path = os.path.join(tmp_dir(), "vr_config4_tree.npz")
+    st.save_npz(path)
     rt = rb.RefTree(path)
     c12 = np.stack([synth.c2w_to_colmajor12(p) for p in poses])
     opt = rb.make_options()
@@ -557,7 +586,7 @@ def main_config4(args, rank, world, local_rank):
     if rank == 0:
         identical = bool(np.array_equal(host[::13].numpy(), solo))
     t0 = time.perf_counter()
-    n_e2e = max(2, min(args.steps, 5))
+    n_e2e = args.steps
     for i in range(n_e2e):
         e2e_step(i)
     te = torch.tensor([(time.perf_counter() - t0) * 1e3 / n_e2e], dtype=torch.float64, device=dev)
@@ -566,6 +595,8 @@ def main_config4(args, rank, world, local_rank):
     e2e_ms = float(te.item())
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"frames": frame_sample(host)})
         peak, peak_note = measured_peak()
         rays = C4_W * C4_H * C4_POSES
         line = {
@@ -609,7 +640,13 @@ def main():
     ap.add_argument("--gather", default="p2p", choices=["p2p", "nccl"], help="N>1: how frames reach rank 0")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cli", action="store_true", help="skip the volrend_headless leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the RGBA8 frames of the last timed step to DIR/<name>.npy as float32 (rank 0; a fixed "
+                         "sample of %d pixels when there are more): frames (batch), frames_e2e (host-buffer leg); "
+                         "config4: frames (reassembled)" % DUMP_PIXELS)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
 
     rank = env_int("RANK", 0)
@@ -728,6 +765,7 @@ def main():
     sync_all()
     launches = lib().vr_launch_count() - launches0
     ms_total = e0.elapsed_time(e1)
+    outputs = {"frames": frame_sample(imgs[(args.steps - 1) & 1])} if args.dump_outputs and rank == 0 else None
     # keep the identical load running (untimed) until the clock sampler has covered >= 1.2 s of it
     extra = 0
     while rank == 0 and world == 1 and time.time() - cs.t0 < 1.2:
@@ -751,7 +789,7 @@ def main():
         render_frames_host(tree, cams, opt, host)
     sync_all()
     t0 = time.perf_counter()
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         render_frames_host(tree, cams, opt, host)
     torch.cuda.synchronize()
@@ -759,6 +797,8 @@ def main():
     if world > 1:
         dist.all_reduce(te, op=dist.ReduceOp.MAX)
     e2e_ms = float(te.item())
+    if outputs is not None:
+        outputs["frames_e2e"] = frame_sample(host)
 
     if rank == 0:
         peak, peak_note = measured_peak()
@@ -813,6 +853,8 @@ def main():
         if not args.no_cpu_baseline and world == 1:
             with StdoutToStderr():
                 line["cpu_baseline"] = cpu_baseline(scene)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

@@ -1,14 +1,13 @@
 """`-m gpu`: parity of the DEFAULT kernel at the sizes bench.py and BASELINE.json quote (VERDICT r1 item 3).
 
-  config 2   depth-10 SH16 bench tree, 800x800      full frames vs the reference kernel (oracle/_ref), bit for bit
+  config 2   depth-10 SH16 bench tree, 800x800      full frames vs the reference kernel, bit for bit
   config 4   depth-11 SH25 tree, 1920x1080           full frame vs the reference kernel; vr_render_bands for 2/4/8 parts
                                                      reassembles to exactly that frame
 
-When oracle/_ref did not travel to the box the same frames are checked against the CPU oracle on windows
-that include the image borders and the silhouette (tolerance 1e-4 required, 2e-6 achieved).  These trees
-exercise what the small cases cannot: 6 levels of wide tables, table ids > 2^17, record offsets > 2^31 bytes."""
-import os
-
+The reference kernel's frames are stored as whole-frame digests plus a pixel sample (tests/golden/frames).
+The same frames are also checked against the CPU oracle on windows that include the image borders and the
+silhouette (tolerance 1e-4 required, 2e-6 achieved).  These trees exercise what the small cases cannot:
+6 levels of wide tables, table ids > 2^17, record offsets > 2^31 bytes."""
 import numpy as np
 import pytest
 
@@ -40,29 +39,14 @@ def _render_default(tree, cam, want_counters=False):
     return fo.cpu().numpy(), img.cpu().numpy(), cnt
 
 
-def _check_against_reference_or_oracle(st, tree, cams, tmp_path, name, windows):
-    """Full frames vs the reference CUDA kernel when oracle/_ref is on the box, else oracle windows."""
+def _check_against_reference_and_oracle(st, tree, cams, names, windows):
+    """Full frames vs the stored frames of the reference CUDA kernel, then the first frame vs oracle windows."""
+    from golden_cases import check_reference_frame
     from oracle import binding as ob
-    from oracle import ref_binding as rb
     frames = [_render_default(tree, c, want_counters=(i == 0)) for i, c in enumerate(cams)]
-    if rb.available():
-        path = str(tmp_path / f"{name}.npz")
-        st.save_npz(path)
-        rt = rb.RefTree(path)
-        try:
-            for (f, u, _), cam in zip(frames, cams):
-                c12 = np.ascontiguousarray(cam.transform, np.float32).reshape(12)
-                fr = rt.render_f32(cam.width, cam.height, cam.fx, cam.fy, c12, rb.make_options())
-                ur = rt.render_u8(cam.width, cam.height, cam.fx, cam.fy, c12, rb.make_options())
-                assert np.abs(f - fr).max() <= TOL
-                assert np.array_equal(f, fr), "float RGBA differs from the reference kernel (expected bit-identical)"
-                assert np.array_equal(u, ur)
-        finally:
-            rt.close()
-        mode = "reference kernel, full frames"
-    else:
-        mode = "CPU oracle windows (oracle/_ref not on this box)"
-    # the oracle windows run in both modes: they also pin the work counters' building blocks
+    for (f, u, _), name in zip(frames, names):
+        check_reference_frame(name, f, u, TOL)
+    # the oracle windows also pin the work counters' building blocks
     ot = ob.OracleTree.from_synth(st)
     f, u, cnt = frames[0]
     cam = cams[0]
@@ -76,10 +60,10 @@ def _check_against_reference_or_oracle(st, tree, cams, tmp_path, name, windows):
         tot["shaded"] += co["shaded"]
     assert tot["samples"] > 0 and tot["shaded"] > 0, "windows must cover the object"
     assert cnt[0] >= tot["samples"] and cnt[2] >= tot["shaded"]
-    return frames, mode
+    return frames
 
 
-def test_config2_bench_tree_800x800_default_kernel(built, tmp_path):
+def test_config2_bench_tree_800x800_default_kernel(built):
     """BASELINE config 2 at full size: the tree bench.py times (depth 10, SH16, seed 0), 800x800."""
     from volrend_b200 import N3Tree, lib, synth
     st = synth.make_tree("lego", depth=10, basis_dim=16, seed=0)
@@ -92,8 +76,7 @@ def test_config2_bench_tree_800x800_default_kernel(built, tmp_path):
     fx = synth.focal_for(800)
     cams = [_cam(800, 800, fx, poses[i]) for i in (0, 77)]
     windows = [(0, 0, 64, 48), (736, 752, 64, 48), (368, 376, 64, 48), (250, 300, 48, 64)]
-    frames, mode = _check_against_reference_or_oracle(st, tree, cams, tmp_path, "bench_tree", windows)
-    print("config 2 parity:", mode)
+    frames = _check_against_reference_and_oracle(st, tree, cams, ["config2_pose0", "config2_pose77"], windows)
     # the batch default (inline shading) and, explicitly, each product kernel on single frames: same bits
     import torch
     from volrend_b200 import RenderOptions, launch_renderer, render_batch
@@ -112,7 +95,7 @@ def test_config2_bench_tree_800x800_default_kernel(built, tmp_path):
             lib().vr_set_variant(0)
 
 
-def test_config4_sh25_depth11_1080p_and_bands(built, tmp_path):
+def test_config4_sh25_depth11_1080p_and_bands(built):
     """BASELINE config 4: depth-11 SH25 tree at 1920x1080, full frame + ray-tile (band) sharding for 2/4/8 GPUs."""
     import torch
     from volrend_b200 import N3Tree, RenderOptions, render_bands, synth
@@ -126,8 +109,7 @@ def test_config4_sh25_depth11_1080p_and_bands(built, tmp_path):
     pose = synth.nerf_synthetic_test_poses(40, radius=1.6, elev_deg=25.0)[7]
     cam = _cam(W, H, fx, pose)
     windows = [(0, 0, 48, 32), (W - 48, H - 32, 48, 32), (900, 500, 64, 48), (600, 700, 48, 32)]
-    frames, mode = _check_against_reference_or_oracle(st, tree, [cam], tmp_path, "config4_tree", windows)
-    print("config 4 parity:", mode)
+    frames = _check_against_reference_and_oracle(st, tree, [cam], ["config4_pose7"], windows)
     f_full, u_full, _ = frames[0]
     for world in (2, 4, 8):
         band_h = 8

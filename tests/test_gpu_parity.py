@@ -1,5 +1,5 @@
 """`-m gpu`: the CUDA path through the C-ABI against (a) the CPU oracle, (b) the golden vectors of
-the reference CUDA kernel, (c) the reference kernel itself when oracle/_ref is on the box, and
+the reference CUDA kernel, (c) stored frames of the reference loader + kernel on tree.npz files, and
 through size-independent properties at the full benchmark size.
 
 Tolerances: float RGBA <= 1e-4 abs per channel (BASELINE.json north_star).  In practice the sample
@@ -145,28 +145,18 @@ def test_golden_vectors_of_reference_kernel(built):
         assert (u != z["ref_u8"]).any(-1).sum() <= 2
 
 
-def test_live_reference_kernel_if_present(built, small_trees, tmp_path):
-    """When oracle/_ref/libvolrend_ref.so travelled to the box: same tree.npz through the
-    reference loader + launch_renderer and through ours."""
-    from oracle import ref_binding as rb
-    if not rb.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    from volrend_b200 import N3Tree, RenderOptions, synth
-    for name in ("sh16_d6", "sh25_d5", "rgba_d5"):
-        st = small_trees[name]
+def test_reference_frames_through_our_loader(built, tmp_path):
+    """The same tree.npz through our loader + kernel vs the stored frames of the reference loader +
+    launch_renderer (tests/golden/frames): bit-identical."""
+    from golden_cases import check_reference_frame, frame_case
+    from volrend_b200 import N3Tree, RenderOptions
+    for name in ("loader_sh16", "loader_sh25", "loader_rgba"):
+        st, W, H, fx, pose = frame_case(name)
         path = str(tmp_path / f"{name}.npz")
         st.save_npz(path)
-        rt = rb.RefTree(path)
-        tree = N3Tree(path)                      # our loader on the same file
-        cam = make_cam(80, 60, synth.nerf_synthetic_test_poses(8)[2])
-        c12 = np.ascontiguousarray(cam.transform, np.float32).reshape(12)
-        fr = rt.render_f32(80, 60, cam.fx, cam.fy, c12, rb.make_options())
-        ur = rt.render_u8(80, 60, cam.fx, cam.fy, c12, rb.make_options())
-        rt.close()
-        f, u, _ = gpu_render(tree, cam, RenderOptions())
-        assert np.abs(f - fr).max() <= TOL
-        assert np.array_equal(f, fr), "float RGBA is expected to be bit-identical to the reference kernel"
-        assert np.array_equal(u, ur)
+        tree = N3Tree(path)
+        f, u, _ = gpu_render(tree, make_cam(W, H, pose), RenderOptions())
+        check_reference_frame(name, f, u, TOL)
 
 
 def test_tiles_batches_and_variants_are_bit_identical(built, dev_trees):
@@ -423,8 +413,9 @@ def test_render_bands_matches_full_frame(built, dev_trees):
 def test_gpu_decode_of_quantised_tree(built, tmp_path):
     """vr_tree_create_quantized (GPU decode of quant_colors/quant_map/sigma/data_retained) gives the
     same device tree as the reference's CPU decode (src/n3tree.cpp:279-340): identical renders,
-    identical probed coefficients, also against the reference loader + kernel when present."""
+    identical probed coefficients, and for SH the stored frames of the reference loader + kernel."""
     torch = _torch()
+    from golden_cases import check_reference_frame
     from volrend_b200 import N3Tree, RenderOptions, lib, synth
     from volrend_b200._capi import check
     for basis, n_retain, fmt in ((16, 1, "SH"), (9, 0, "SH"), (7, 2, "SG")):
@@ -446,13 +437,8 @@ def test_gpu_decode_of_quantised_tree(built, tmp_path):
             check(lib().vr_probe_lumisphere(t_cpu._handle, arr, out_c.data_ptr(), None))
             torch.cuda.synchronize()
             assert torch.equal(out_g, out_c)
-        from oracle import ref_binding as rb
-        if rb.available() and fmt == "SH":
-            rt = rb.RefTree(path)                       # reference loader decodes on the CPU
-            c12 = np.ascontiguousarray(cam.transform, np.float32).reshape(12)
-            fr = rt.render_f32(96, 80, cam.fx, cam.fy, c12, rb.make_options())
-            rt.close()
-            assert np.array_equal(fg, fr)
+        if fmt == "SH":                                 # the reference loader decodes on the CPU
+            check_reference_frame(f"quant_sh{basis}", fg, ug, TOL)
 
 
 def test_png_egress_api_and_cli(built, dev_trees, small_trees, tmp_path):
