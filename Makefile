@@ -1,6 +1,7 @@
 # Build of the B200-native volrend backend.  No GPU is needed to build (nvcc cross-compiles).
 #   make lib      volrend_b200/libvolrend_b200.so   the product: C-ABI + sm_100a kernels
 #   make oracle   oracle/liboracle.so               CPU restatement (test infrastructure)
+#                 oracle/libray_oracle.so           + its ray-batch entry points
 #   make ref      oracle/_ref/*                     the unmodified reference, built from
 #                                                   $(VOLREND_REF) (only when it exists)
 #   make shim     build/volrend_headless ...        reference CLI linked against OUR backend
@@ -40,6 +41,10 @@ $(OBJ)/vr_api.o: volrend_b200/csrc/vr_api.cu volrend_b200/csrc/vr_types.h volren
 	@mkdir -p $(OBJ)
 	$(NVCC) $(NVFLAGS) -c $< -o $@
 
+$(OBJ)/vr_rays.o: volrend_b200/csrc/vr_rays.cu volrend_b200/csrc/vr_march.cuh volrend_b200/csrc/vr_types.h volrend_b200/csrc/vr_kernels.h include/volrend_b200.h
+	@mkdir -p $(OBJ)
+	$(NVCC) $(NVFLAGS) -c $< -o $@
+
 $(OBJ)/vr_mg.o: volrend_b200/csrc/vr_mg.cu include/volrend_b200.h
 	@mkdir -p $(OBJ)
 	$(NVCC) $(NVFLAGS) -c $< -o $@
@@ -48,15 +53,18 @@ $(OBJ)/vr_png.o: volrend_b200/csrc/vr_png.cpp include/volrend_b200.h
 	@mkdir -p $(OBJ)
 	$(CXX) -O3 -std=c++17 -fPIC -Iinclude -c $< -o $@
 
-$(LIB): $(OBJ)/vr_api.o $(OBJ)/vr_mg.o $(OBJ)/vr_png.o $(KOBJS)
+$(LIB): $(OBJ)/vr_api.o $(OBJ)/vr_mg.o $(OBJ)/vr_png.o $(OBJ)/vr_rays.o $(KOBJS)
 	$(NVCC) $(ARCH) -shared -o $@ $^ -lz -lpthread
 
-oracle: oracle/liboracle.so
+oracle: oracle/liboracle.so oracle/libray_oracle.so
 oracle/liboracle.so: oracle/march_oracle.c oracle/march_oracle.h
+	$(CC) -O2 -ffp-contract=off -fno-fast-math -fPIC -shared -pthread -o $@ $< -lm
+oracle/libray_oracle.so: oracle/ray_oracle.c oracle/ray_oracle.h oracle/march_oracle.c oracle/march_oracle.h
 	$(CC) -O2 -ffp-contract=off -fno-fast-math -fPIC -shared -pthread -o $@ $< -lm
 
 ref:
-	@if [ -d "$(VOLREND_REF)/src/cuda" ]; then $(MAKE) -C oracle -f Makefile.ref VOLREND_REF=$(VOLREND_REF); \
+	@if [ -d "$(VOLREND_REF)/src/cuda" ]; then $(MAKE) -C oracle -f Makefile.ref VOLREND_REF=$(VOLREND_REF) && \
+	 $(MAKE) -C oracle -f Makefile.rays VOLREND_REF=$(VOLREND_REF); \
 	 else echo "reference tree $(VOLREND_REF) not present: using prebuilt oracle/_ref if any"; fi
 
 shim:
@@ -64,4 +72,4 @@ shim:
 	 else echo "reference tree $(VOLREND_REF) not present: shim needs the reference headers"; fi
 
 clean:
-	rm -rf build $(LIB) oracle/liboracle.so oracle/_ref
+	rm -rf build $(LIB) oracle/liboracle.so oracle/libray_oracle.so oracle/_ref

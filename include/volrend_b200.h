@@ -17,6 +17,8 @@
  *                                      colour + depth inputs (volrend.cu:92-96,143-146)
  *   vr_render_batch                    the per-pose loop of main_headless.cpp:208-223 as
  *                                      one call (same per-view semantics)
+ *   vr_render_rays / vr_camera_rays    caller-supplied ray batches (origins + directions in,
+ *                                      float RGBA out) on the same march kernels
  *   vr_render_frames_host              main_headless.cpp:208-223 with `-o`: renders and
  *                                      copies every frame to host memory (:216-219)
  *   vr_probe_lumisphere                retrieve_cursor_lumisphere_kernel (volrend.cu:175-191)
@@ -159,6 +161,29 @@ int vr_band_rows(int height, int band_h, int n_parts, int part);
 /* Same for n_views cameras in ONE launch: view i's bands land at rgba8_dev + i * 4*width*vr_band_rows(). */
 int vr_render_bands_batch(const vr_tree* tree, const vr_camera* cams, int n_views, const vr_options* opt, int band_h,
                           int n_parts, int part, uint8_t* rgba8_dev, float* rgba32f_dev, void* stream);
+
+/* Ray batches: renders n_rays caller-supplied rays instead of the pixels of a camera.
+ *   origins_dev, dirs_dev  device float32 [n_rays][3], world space; directions need not be unit length
+ *   t_max_dev              device float32 [n_rays] depth limits, or NULL (= 1e9 for every ray)
+ *   rgba32f_dev            device float4 [n_rays]: premultiplied RGB + background, alpha
+ *   counters_dev           device vr_counters to accumulate into, or NULL
+ * Ray i is rendered exactly as render_kernel renders a pixel (volrend.cu:136-158, offscreen branch) with
+ * screen2worlddir replaced by the loaded ray: the direction is normalised with screen2worlddir's _normalize and kept
+ * as the view direction of the basis, then maybe_world2ndc, the tree's offset/scale, rodrigues(rot_dirs) and trace_ray
+ * with t_max[i] as depth limit -- the unit of the composite-mode depth (rt_core.cuh:77): for non-NDC trees the world
+ * distance from the origin along the normalised direction.  The result is composited over background_brightness.
+ * Every vr_options field applies.  A ray with a non-finite origin or direction component, or whose direction has
+ * fp32 length 0 or infinity, is a miss: background with alpha 0 (alpha 1 under render_depth, as for every miss), not
+ * counted in rays_hit.  Any leading shape of rays is the caller's; n_rays == 0 is a no-op.  Runs on the tree's batch
+ * kernel variant (vr_tree_variant; vr_set_variant 7 selects the shading queue); other variants fail with
+ * VR_EUNSUPPORTED.  The ray arrays may be written by the previous kernel on `stream` without synchronisation.
+ *
+ * vr_camera_rays writes the rays the march generates for `cam` (tile NULL = full frame), one per pixel, row-major
+ * over the tile: origin c2w[9..11], direction the un-normalised _mv3(c2w, xyz) of screen2worlddir.  Fed to
+ * vr_render_rays they reproduce vr_render's float output and work counters bit for bit. */
+int vr_render_rays(const vr_tree* tree, const float* origins_dev, const float* dirs_dev, const float* t_max_dev,
+                   int n_rays, const vr_options* opt, float* rgba32f_dev, vr_counters* counters_dev, void* stream);
+int vr_camera_rays(const vr_camera* cam, const vr_rect* tile, float* origins_dev, float* dirs_dev, void* stream);
 
 /* Host-buffer entry point: renders n_views full frames and copies each to
  * rgba8_host + i*4*w*h (pinned or pageable); returns after the last copy completed. */

@@ -74,6 +74,9 @@ SYMBOLS = {
                                       C.POINTER(vr_rect), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "vr_render_surface": (C.c_int, [C.c_void_p, C.POINTER(vr_camera), C.POINTER(vr_options),
                                     C.c_ulonglong, C.c_ulonglong, C.c_void_p]),
+    "vr_render_rays": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(vr_options),
+                                 C.c_void_p, C.c_void_p, C.c_void_p]),
+    "vr_camera_rays": (C.c_int, [C.POINTER(vr_camera), C.POINTER(vr_rect), C.c_void_p, C.c_void_p, C.c_void_p]),
     "vr_render_frames_host": (C.c_int, [C.c_void_p, C.POINTER(vr_camera), C.c_int, C.POINTER(vr_options),
                                         C.c_void_p]),
     "vr_write_png": (C.c_int, [C.c_char_p, C.c_void_p, C.c_int, C.c_int]),

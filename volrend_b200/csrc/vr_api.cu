@@ -745,7 +745,8 @@ int stream_res(vr_tree* t, cudaStream_t stream, StreamRes*& out) {
     return VR_OK;
 }
 
-int dispatch(const vr_tree* t, LaunchDev& P, bool count, bool surface, cudaStream_t stream) {
+// rays: P describes caller-supplied rays (launch_rays) instead of pixels of a camera (launch_march)
+int dispatch(const vr_tree* t, LaunchDev& P, bool count, bool surface, cudaStream_t stream, bool rays = false) {
     LaunchCfg cfg;
     cfg.variant = vr_get_variant();
     if (!variant_ok(t->dev.kbd, cfg.variant))
@@ -784,14 +785,17 @@ int dispatch(const vr_tree* t, LaunchDev& P, bool count, bool surface, cudaStrea
     cfg.pdl = !no_pdl;
     cudaError_t e;
     switch (t->dev.kbd) {
-        case -1: e = launch_march<-1>(P, cfg); break;
-        case 1: e = launch_march<1>(P, cfg); break;
-        case 4: e = launch_march<4>(P, cfg); break;
-        case 9: e = launch_march<9>(P, cfg); break;
-        case 16: e = launch_march<16>(P, cfg); break;
-        case 25: e = launch_march<25>(P, cfg); break;
+        case -1: e = rays ? launch_rays<-1>(P, cfg) : launch_march<-1>(P, cfg); break;
+        case 1: e = rays ? launch_rays<1>(P, cfg) : launch_march<1>(P, cfg); break;
+        case 4: e = rays ? launch_rays<4>(P, cfg) : launch_march<4>(P, cfg); break;
+        case 9: e = rays ? launch_rays<9>(P, cfg) : launch_march<9>(P, cfg); break;
+        case 16: e = rays ? launch_rays<16>(P, cfg) : launch_march<16>(P, cfg); break;
+        case 25: e = rays ? launch_rays<25>(P, cfg) : launch_march<25>(P, cfg); break;
         default: return fail(VR_EUNSUPPORTED, "unsupported kernel basis %d", t->dev.kbd);
     }
+    if (e == cudaErrorNotSupported)
+        return fail(VR_EUNSUPPORTED, "kernel variant %d has no ray-batch form (ray launches run on variants 0, 7 and %d)",
+                    cfg.variant, kVariantInline);
     if (e != cudaSuccess) return fail(VR_ECUDA, "kernel launch failed: %s", cudaGetErrorString(e));
     g_launches += 1;
     return VR_OK;
@@ -955,6 +959,55 @@ int vr_debug_trace(const vr_tree* t, const vr_camera* cam, const vr_options* opt
     P.x0 = 0; P.y0 = 0; P.w = r.w; P.h = r.h;
     P.rgba8 = rgba8_dev; P.counters = counters_dev; P.trace = trace_dev;
     return dispatch(t, P, true, false, (cudaStream_t)stream_);
+}
+
+int vr_render_rays(const vr_tree* t, const float* origins_dev, const float* dirs_dev, const float* t_max_dev, int n_rays,
+                   const vr_options* opt, float* rgba32f_dev, vr_counters* counters_dev, void* stream_) {
+    if (!t || !opt) return fail(VR_EINVAL, "null argument");
+    if (n_rays < 0) return fail(VR_EINVAL, "n_rays < 0");
+    if (n_rays == 0) return VR_OK;
+    if (!origins_dev || !dirs_dev || !rgba32f_dev) return fail(VR_EINVAL, "null ray or output array");
+    int ndev = 0, dev = -1;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0 || cudaGetDevice(&dev) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(VR_ENODEVICE, "no CUDA device: volrend_b200 has no CPU fallback");
+    }
+    if (dev != t->device) return fail(VR_EINVAL, "tree lives on device %d but device %d is current", t->device, dev);
+    // the product kernels only: the experiment kernels and the ray-pool kernel (kind 8) march pixels of a camera
+    const int v = vr_get_variant();
+    if (v != 0 && v != kVariantQueue && v != kVariantInline)
+        return fail(VR_EUNSUPPORTED, "kernel variant %d has no ray-batch form (ray launches run on variants 0, 7 and %d)", v,
+                    kVariantInline);
+    LaunchDev P{};
+    P.tree = t->dev;
+    fill_opt(P.opt, opt);
+    P.n_views = 1;
+    P.rgbaf = reinterpret_cast<float4*>(rgba32f_dev);
+    P.counters = counters_dev;
+    P.ray_o = origins_dev; P.ray_d = dirs_dev; P.ray_tmax = t_max_dev; P.n_rays = n_rays;
+    return dispatch(t, P, counters_dev != nullptr, false, (cudaStream_t)stream_, true);
+}
+
+int vr_camera_rays(const vr_camera* cam, const vr_rect* tile, float* origins_dev, float* dirs_dev, void* stream_) {
+    if (!cam || !origins_dev || !dirs_dev) return fail(VR_EINVAL, "null argument");
+    if (cam->width <= 0 || cam->height <= 0) return fail(VR_EINVAL, "bad camera size %dx%d", cam->width, cam->height);
+    vr_rect r{0, 0, cam->width, cam->height};
+    if (tile) {
+        r = *tile;
+        if (r.w < 0 || r.h < 0 || r.x0 < 0 || r.y0 < 0 || r.x0 + r.w > cam->width || r.y0 + r.h > cam->height)
+            return fail(VR_EINVAL, "tile (%d,%d,%d,%d) outside %dx%d frame", r.x0, r.y0, r.w, r.h, cam->width, cam->height);
+    }
+    if (r.w == 0 || r.h == 0) return VR_OK;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(VR_ENODEVICE, "no CUDA device: volrend_b200 has no CPU fallback");
+    }
+    CamDev c;
+    fill_cam(c, cam);
+    VR_CUDA(launch_camera_rays(c, r.x0, r.y0, r.w, r.h, origins_dev, dirs_dev, (cudaStream_t)stream_));
+    g_launches += 1;
+    return VR_OK;
 }
 
 int vr_render(const vr_tree* t, const vr_camera* cam, const vr_options* opt, const vr_rect* tile, uint8_t* rgba8_dev,

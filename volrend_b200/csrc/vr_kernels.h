@@ -33,16 +33,32 @@ cudaError_t launch_march(LaunchDev& P, const LaunchCfg& cfg);
 template <int KBD>
 bool variant_supported(int variant);
 
+// Caller-supplied rays (P.ray_o / ray_d / ray_tmax, P.n_rays > 0, float4 output in P.rgbaf): variant 0 (the batch
+// default, inline shading) or 7 (shading queue, >= 4 basis functions); cudaErrorNotSupported for any other variant.
+template <int KBD>
+cudaError_t launch_rays(LaunchDev& P, const LaunchCfg& cfg);
+
+// vr_camera_rays: the rays the march generates for the pixels of tile (x0, y0, w, h) of `cam`, row-major:
+// origins c2w[9..11], directions before normalisation (vr_march.cuh camera_ray_dir).  float [w*h][3] each.
+cudaError_t launch_camera_rays(const CamDev& cam, int x0, int y0, int w, int h, float* origins, float* dirs,
+                               cudaStream_t stream);
+
 // bytes of parked-ray storage a kind-8 launch needs on a device with num_sms SMs (0 when KBD has no such kernel)
 template <int KBD>
 size_t pool_bytes_for(int num_sms, int max_depth);
 
 extern template cudaError_t launch_march<-1>(LaunchDev&, const LaunchCfg&);
+extern template cudaError_t launch_rays<-1>(LaunchDev&, const LaunchCfg&);
 extern template cudaError_t launch_march<1>(LaunchDev&, const LaunchCfg&);
+extern template cudaError_t launch_rays<1>(LaunchDev&, const LaunchCfg&);
 extern template cudaError_t launch_march<4>(LaunchDev&, const LaunchCfg&);
+extern template cudaError_t launch_rays<4>(LaunchDev&, const LaunchCfg&);
 extern template cudaError_t launch_march<9>(LaunchDev&, const LaunchCfg&);
+extern template cudaError_t launch_rays<9>(LaunchDev&, const LaunchCfg&);
 extern template cudaError_t launch_march<16>(LaunchDev&, const LaunchCfg&);
+extern template cudaError_t launch_rays<16>(LaunchDev&, const LaunchCfg&);
 extern template cudaError_t launch_march<25>(LaunchDev&, const LaunchCfg&);
+extern template cudaError_t launch_rays<25>(LaunchDev&, const LaunchCfg&);
 extern template bool variant_supported<-1>(int);
 extern template size_t pool_bytes_for<-1>(int, int);
 extern template bool variant_supported<1>(int);

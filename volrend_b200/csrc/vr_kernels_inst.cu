@@ -7,6 +7,7 @@
 //   kind 8           (VR_EXPERIMENTS) the same kernel with the ray pool (POOL = true): measured, slower
 //   kind 3, tune 193 march_persistent_kernel with inline shading: default for batches and for RGBA / 1 / 25 basis
 //                    functions, and the A/B partner of the queue kernel in the parity tests and the bench
+// Both product kernels are also instantiated with OUT = kOutRays for caller-supplied rays (launch_rays).
 // Built only with -DVR_EXPERIMENTS (make lib SUFFIX=_exp EXTRA=-DVR_EXPERIMENTS): the measured and
 // rejected structures of round 1 -- CTA-per-tile kernel, TMA-staged top grid, deferred shading,
 // software-pipelined march, tuning knobs (DESIGN.md 4).
@@ -71,9 +72,19 @@ void set_work(LaunchDev& P, const LaunchCfg& cfg, bool blocks = true) {
     set_div((uint32_t)P.tiles_x, P.div_row_mul, P.div_row_shift);
 }
 
+// Ray launches: work item k = rays 32k .. 32k+31, one item per queue pull (blocks of tiles are a 2-D pixel notion).
+// The queue kernel carries an item as (lane << 26 | item): items of n_rays <= 2^31 - 1 rays stay below 2^26.
+static_assert((0x7fffffffLL + 31) / 32 <= (1LL << 26), "ray items must fit the 26-bit item field");
+void set_work_rays(LaunchDev& P, const LaunchCfg& cfg) {
+    P.work_counter = cfg.queue;
+    P.blk_mode = 0; P.blocks_x = 0; P.n_blocks = 0;
+    P.n_tiles = (int)(((long long)P.n_rays + 31) / 32);
+}
+
 template <typename K>
 cudaError_t launch_persistent_grid(K kernel, size_t smem, LaunchDev& P, const LaunchCfg& cfg, bool blocks = true) {
-    set_work(P, cfg, blocks);
+    if (P.n_rays > 0) set_work_rays(P, cfg);
+    else set_work(P, cfg, blocks);
     int grid = resident_ctas(kernel, smem, cfg.num_sms);
     if (cfg.max_ctas > 0 && grid > cfg.max_ctas) grid = cfg.max_ctas;
     const int need = (P.n_tiles + (kBlock / 32) - 1) / (kBlock / 32);
@@ -230,6 +241,20 @@ cudaError_t launch_march(LaunchDev& P, const LaunchCfg& cfg) {
     return cudaErrorInvalidValue;
 }
 
+// Ray launches (vr_render_rays): the two product kernels only.  Variant 0 resolves to the batch default, the inline
+// kernel (vr_tree_variant); 7 selects the shading queue.  Anything else: cudaErrorNotSupported.
+template <int KBD>
+cudaError_t launch_rays(LaunchDev& P, const LaunchCfg& cfg) {
+    const int variant = cfg.variant == 0 ? 3 + 16 * kInline : cfg.variant;
+    if (P.n_rays <= 0 || cfg.surface) return cudaErrorInvalidValue;
+    if (variant == 7 && KBD >= 4)
+        return cfg.count ? launch_queue<KBD, true, kOutRays>(P, cfg) : launch_queue<KBD, false, kOutRays>(P, cfg);
+    if (variant == 3 + 16 * kInline)
+        return cfg.count ? launch_persistent<KBD, false, true, kOutRays, kInline>(P, cfg)
+                         : launch_persistent<KBD, false, false, kOutRays, kInline>(P, cfg);
+    return cudaErrorNotSupported;
+}
+
 template <int KBD>
 size_t pool_bytes_for(int num_sms, int max_depth) {
 #ifndef VR_EXPERIMENTS
@@ -246,6 +271,7 @@ size_t pool_bytes_for(int num_sms, int max_depth) {
 }
 
 template cudaError_t launch_march<VR_KBD>(LaunchDev&, const LaunchCfg&);
+template cudaError_t launch_rays<VR_KBD>(LaunchDev&, const LaunchCfg&);
 template size_t pool_bytes_for<VR_KBD>(int, int);
 template bool variant_supported<VR_KBD>(int);
 

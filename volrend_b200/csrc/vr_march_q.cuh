@@ -234,6 +234,21 @@ __device__ __forceinline__ void pool_unlock(uint32_t lock_addr) {
 // shared memory of one CTA: [ control 16 B | parked ray constants | basis values | shading queues | table-id stacks ]
 constexpr uint32_t kCtrlBytes = 16;
 
+// Basis values of this lane's ray (view direction vd) -> shared memory, bs[q][lane].
+template <int KBD>
+__device__ __forceinline__ void park_basis_q(const LaunchDev& P, const float (&vd)[3], uint32_t bs_warp, int lane) {
+    float B[BasisCount<KBD>::n];
+    eval_basis<KBD>(P.tree, P.opt, vd, B);
+#pragma unroll
+    for (int q = 0; q < BasisQ<KBD>::n; ++q) {
+        float v[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) v[k] = (4 * q + k < BasisCount<KBD>::n) ? B[4 * q + k] : 0.f;
+        sts128_a(bs_warp + ((uint32_t)q * 32u + (uint32_t)lane) * 16u, __float_as_uint(v[0]), __float_as_uint(v[1]),
+                 __float_as_uint(v[2]), __float_as_uint(v[3]));
+    }
+}
+
 // ---------------------------------------------------------------- the kernel
 template <int KBD, bool COUNT, int OUT, bool POOL = false>
 __global__ void __launch_bounds__(kBlock, kMinBlocks) march_queue_kernel(const __grid_constant__ LaunchDev P) {
@@ -266,7 +281,9 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks) march_queue_kernel(const _
     pdl_launch_dependents();
     Counts cnt = {0, 0, 0, 0, 0};
     bool dep_done = false;
-    if (COUNT || P.cams) {  // instrumented runs and batches (camera ring written by a copy) do not overlap
+    // instrumented runs, batches (camera ring written by a copy) and ray launches (ray arrays usually written by the
+    // previous kernel of the stream) do not overlap
+    if (COUNT || P.cams || OUT == kOutRays) {
         pdl_wait_predecessor();
         dep_done = true;
     }
@@ -350,40 +367,39 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks) march_queue_kernel(const _
                 }
                 break;
             }
-            int view, tx, ty;
-            decode_item<false>(P, item, view, tx, ty);
-            const int lx = tx * kTW + (lane % kTW), ly = ty * kTH + (lane / kTW);
-            const bool inb = lx < P.w && ly < P.h;
-            const CamDev& cam = P.cams ? P.cams[view] : P.cam;
-            if (COUNT && P.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_begin));
-
-            const int px = P.x0 + lx, py = P.y0 + frame_row(P, ly);
-            float tlim = 1e9f;
-            if (P.composite && inb) {  // volrend.cu:92-96,143-146
-                if (!dep_done) { pdl_wait_predecessor(); dep_done = true; }  // reads the previous image
-                const size_t o = ((size_t)view * P.h + ly) * P.w + lx;
-                if (OUT == kOutSurface) {
-                    init = surf2Dread<uint32_t>(P.surf, px * 4, py, cudaBoundaryModeZero);
-                    if (P.dsurf) tlim = surf2Dread<float>(P.dsurf, px * 4, py, cudaBoundaryModeZero);
-                } else {
-                    init = reinterpret_cast<const uint32_t*>(P.rgba8)[o];
-                    if (P.depth_in) tlim = P.depth_in[o];
+            if constexpr (OUT == kOutRays) {   // lane l of item k: ray 32k + l
+                const uint32_t ray = item * 32u + (uint32_t)lane;
+                float c[3], d[3], tlim;
+                if (ray < (uint32_t)P.n_rays && P.tree.N > 0 && load_ray(P, ray, c, d, tlim)) {
+                    float vd[3];
+                    hit = ray_geometry_world(P.tree, P.opt, d[0], d[1], d[2], c, tlim, R, vd, P.tree.pos_scale);
+                    if (hit) park_basis_q<KBD>(P, vd, bs_warp, lane);
                 }
-            }
-            if (inb && P.tree.N > 0) {
-                float vd[3];
-                hit = ray_geometry(P.tree, P.opt, cam, px, py, tlim, R, vd, P.tree.pos_scale);
-                if (hit) {  // basis values of this ray -> shared memory, bs[q][lane]
-                    float B[BasisCount<KBD>::n];
-                    eval_basis<KBD>(P.tree, P.opt, vd, B);
-#pragma unroll
-                    for (int q = 0; q < KQ; ++q) {
-                        float v[4];
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) v[k] = (4 * q + k < BasisCount<KBD>::n) ? B[4 * q + k] : 0.f;
-                        sts128_a(bs_warp + ((uint32_t)q * 32u + (uint32_t)lane) * 16u, __float_as_uint(v[0]), __float_as_uint(v[1]),
-                                 __float_as_uint(v[2]), __float_as_uint(v[3]));
+            } else {
+                int view, tx, ty;
+                decode_item<false>(P, item, view, tx, ty);
+                const int lx = tx * kTW + (lane % kTW), ly = ty * kTH + (lane / kTW);
+                const bool inb = lx < P.w && ly < P.h;
+                const CamDev& cam = P.cams ? P.cams[view] : P.cam;
+                if (COUNT && P.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_begin));
+
+                const int px = P.x0 + lx, py = P.y0 + frame_row(P, ly);
+                float tlim = 1e9f;
+                if (P.composite && inb) {  // volrend.cu:92-96,143-146
+                    if (!dep_done) { pdl_wait_predecessor(); dep_done = true; }  // reads the previous image
+                    const size_t o = ((size_t)view * P.h + ly) * P.w + lx;
+                    if (OUT == kOutSurface) {
+                        init = surf2Dread<uint32_t>(P.surf, px * 4, py, cudaBoundaryModeZero);
+                        if (P.dsurf) tlim = surf2Dread<float>(P.dsurf, px * 4, py, cudaBoundaryModeZero);
+                    } else {
+                        init = reinterpret_cast<const uint32_t*>(P.rgba8)[o];
+                        if (P.depth_in) tlim = P.depth_in[o];
                     }
+                }
+                if (inb && P.tree.N > 0) {
+                    float vd[3];
+                    hit = ray_geometry(P.tree, P.opt, cam, px, py, tlim, R, vd, P.tree.pos_scale);
+                    if (hit) park_basis_q<KBD>(P, vd, bs_warp, lane);
                 }
             }
             if (COUNT && hit) ++cnt.hit;
@@ -597,6 +613,28 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks) march_queue_kernel(const _
         // this lane's pixel: its own tile, or the tile a parked ray came from
         uint32_t packed;
         asm volatile("ld.shared.u32 %0, [%1];" : "=r"(packed) : "r"(rs + 2u * kBlock * 16u + 12u) : "memory");
+        if constexpr (OUT == kOutRays) {   // this lane's ray: 32 * item + lane slot (offscreen compositing only)
+            const uint32_t ray = (packed & 0x3ffffffu) * 32u + (packed >> 26);
+            if (packed != 0xffffffffu && ray < (uint32_t)P.n_rays) {
+                float out[4] = {0.f, 0.f, 0.f, 0.f};
+                if (__float_as_uint(t) != 0x7fc00000u) {   // marched (degenerate rays and misses kept the plain NaN)
+                    if (P.opt.render_depth) r = g = b = fminf(r * 0.3f, 1.0f);  // :177-179,189-191
+                    if (stopped) {  // :181-184
+                        const float sc = __frcp_rn(__fsub_rn(1.f, T));
+                        out[0] = __fmul_rn(r, sc); out[1] = __fmul_rn(g, sc); out[2] = __fmul_rn(b, sc); out[3] = 1.f;
+                    } else {
+                        out[0] = r; out[1] = g; out[2] = b;
+                        out[3] = P.opt.render_depth ? 1.f : __fsub_rn(1.f, T);
+                    }
+                } else if (P.opt.render_depth) {
+                    out[3] = 1.f;  // rt_core.cuh:90-91
+                }
+                const float remain = __fmul_rn(__fsub_rn(1.f, out[3]), P.opt.background_brightness);
+                P.rgbaf[ray] = make_float4(__fadd_rn(remain, out[0]), __fadd_rn(remain, out[1]), __fadd_rn(remain, out[2]), out[3]);
+            }
+            __syncwarp();
+            continue;
+        }
         int view, tx, ty;
         decode_item<false>(P, packed & 0x3ffffffu, view, tx, ty);
         const int lx = tx * kTW + (int)((packed >> 26) % kTW), ly = ty * kTH + (int)((packed >> 26) / kTW);

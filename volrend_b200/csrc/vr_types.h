@@ -128,6 +128,12 @@ struct LaunchDev {
     int32_t blk_mode, blocks_x, n_blocks;
     unsigned char* pool;                // ray-pool kernels: parked-ray stacks, one per CTA (vr_march_q.cuh); nullptr = no parking
     unsigned long long* trace;          // diagnostics: per work item {start ns, end ns, smid, warp}
+    // Ray launches (OUT == kOutRays, vr_render_rays): work item k is the 32 rays 32k .. 32k+31, lane l marches ray
+    // 32k + l (< n_rays) and writes rgbaf[ray].  World-space origins / directions [n_rays][3]; depth limits or nullptr.
+    const float* ray_o;
+    const float* ray_d;
+    const float* ray_tmax;
+    int32_t n_rays;
 };
 
 }  // namespace vrb

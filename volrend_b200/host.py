@@ -253,6 +253,8 @@ class N3Tree:
             check(lib().vr_tree_create(C.byref(d), C.byref(h)))
         self._handle = h
         self._cuda_loaded = True
+        import torch
+        self._device = torch.cuda.current_device()    # the tree lives on the device current at creation
 
     def _plain_desc(self):
         """vr_tree_desc over the decoded host arrays (keeps them alive through the returned tuple)."""
@@ -476,6 +478,69 @@ def render_batch(tree: N3Tree, cams, options: RenderOptions, images, *, float_ou
                                 images.data_ptr() if images is not None else None,
                                 float_out.data_ptr() if float_out is not None else None,
                                 counters.data_ptr() if counters is not None else None, _stream_ptr(stream)))
+
+
+def _check_rays(name, t, last, device=None, shape=None):
+    """ValueError unless ``t`` is a contiguous float32 CUDA tensor [..., last] (on ``device``, of leading ``shape``)."""
+    import torch
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise ValueError(f"{name} must be a CUDA tensor")
+    if t.dtype != torch.float32:
+        raise ValueError(f"{name} must be float32, got {t.dtype}")
+    if not t.is_contiguous():
+        raise ValueError(f"{name} must be contiguous")
+    if last is not None and (t.dim() < 1 or t.shape[-1] != last):
+        raise ValueError(f"{name} must have shape [..., {last}], got {tuple(t.shape)}")
+    lead = tuple(t.shape[:-1]) if last is not None else tuple(t.shape)
+    if shape is not None and lead != tuple(shape):
+        raise ValueError(f"{name} has leading shape {lead}, expected {tuple(shape)}")
+    if device is not None and t.device.index != device:
+        raise ValueError(f"{name} is on cuda:{t.device.index}, expected cuda:{device}")
+    return lead
+
+
+def render_rays(tree: N3Tree, origins, dirs, options: RenderOptions, out, *, t_max=None, counters=None,
+                stream=None) -> None:
+    """Renders caller-supplied rays (``vr_render_rays``): ``origins`` and ``dirs`` float32 CUDA tensors [..., 3] in
+    world space (directions of any non-zero length), ``out`` float32 [..., 4] receives premultiplied RGB + background
+    and alpha per ray; ``t_max`` optional float32 [...] depth limits (world distance along the normalised direction
+    for non-NDC trees).  Each ray is rendered exactly as ``launch_renderer`` renders a pixel, so the rays of
+    :func:`camera_rays` reproduce its float output bit for bit.  Rays with non-finite values or a zero direction are
+    misses (background, alpha 0).  Asynchronous on ``stream``."""
+    if not tree.is_cuda_loaded():
+        raise RuntimeError("N3Tree is not loaded on the device")
+    dev = tree._device
+    lead = _check_rays("origins", origins, 3, dev)
+    _check_rays("dirs", dirs, 3, dev, lead)
+    _check_rays("out", out, 4, dev, lead)
+    if t_max is not None:
+        _check_rays("t_max", t_max, None, dev, lead)
+    n = 1
+    for k in lead:
+        n *= int(k)
+    if n > 0x7fffffff:
+        raise ValueError(f"{n} rays: at most 2^31 - 1 per call")
+    if counters is not None and (not counters.is_cuda or counters.device.index != dev):
+        raise ValueError(f"counters must be a CUDA tensor on cuda:{dev}")
+    o = options._as_c()
+    check(lib().vr_render_rays(tree._handle, origins.data_ptr(), dirs.data_ptr(),
+                               t_max.data_ptr() if t_max is not None else None, n, C.byref(o), out.data_ptr(),
+                               counters.data_ptr() if counters is not None else None, _stream_ptr(stream)))
+
+
+def camera_rays(cam: Camera, origins, dirs, *, tile=None, stream=None) -> None:
+    """The rays the march generates for ``cam`` (``vr_camera_rays``): one per pixel of ``tile`` (x0,y0,w,h; None =
+    full frame), row-major, into float32 CUDA tensors [..., 3] with w*h rays (e.g. [h, w, 3]).  Origins are the
+    camera centre, directions are not normalised.  Asynchronous on ``stream``."""
+    w, h = (cam.width, cam.height) if tile is None else (int(tile[2]), int(tile[3]))
+    lead = _check_rays("origins", origins, 3)
+    _check_rays("dirs", dirs, 3, origins.device.index, lead)
+    if origins.numel() != 3 * w * h:
+        raise ValueError(f"origins/dirs hold {origins.numel() // 3} rays, the {w}x{h} tile has {w * h}")
+    import torch
+    c = cam._as_c()
+    with torch.cuda.device(origins.device):
+        check(lib().vr_camera_rays(C.byref(c), _rect(tile), origins.data_ptr(), dirs.data_ptr(), _stream_ptr(stream)))
 
 
 def render_frames_host(tree: N3Tree, cams, options: RenderOptions, host_images) -> None:
