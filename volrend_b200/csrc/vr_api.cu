@@ -263,7 +263,8 @@ __global__ void table_flag_kernel(const int* __restrict__ depth, long long capac
 }
 
 // wide[table * E + e], E = 8^kWideLv: e = ex << 2*LV | ey << LV | ez holds kWideLv octree levels per axis, first level
-// in the high bit.  The tree hangs v levels below a virtual root (octant 0 each time), so the root table resolves only
+// in the high bit.  A non-leaf entry holds the child table's first entry index, table * E, so that the march forms an
+// entry index as word | e.  The tree hangs v levels below a virtual root (octant 0 each time), so the root table resolves only
 // kWideLv - v real levels: its entries with a non-zero virtual bit are never looked up.
 __global__ void build_wide_kernel(const uint32_t* __restrict__ nodes, const int* __restrict__ depth,
                                   const uint32_t* __restrict__ tid, uint32_t* __restrict__ wide,
@@ -294,7 +295,7 @@ __global__ void build_wide_kernel(const uint32_t* __restrict__ nodes, const int*
         node = w;
         ++dn;
     }
-    wide[o] = tid[node];
+    wide[o] = tid[node] * (uint32_t)kWideEntries;   // the child table's first entry: entry index = word | entry
     wslot[o] = 0xffffffffu;
 }
 
@@ -391,7 +392,7 @@ __global__ void probe_kernel(TreeDev tree, float x, float y, float z, int n_out,
     constexpr uint32_t M = (1u << kWideLv) - 1u;
     for (int j = 0; j < 16; ++j) {
         const int sh = (24 - kWideLv) - kWideLv * j;
-        eidx = T * (uint32_t)kWideEntries + ((((u[0] >> sh) & M) << (2 * kWideLv)) | (((u[1] >> sh) & M) << kWideLv) | ((u[2] >> sh) & M));
+        eidx = T + ((((u[0] >> sh) & M) << (2 * kWideLv)) | (((u[1] >> sh) & M) << kWideLv) | ((u[2] >> sh) & M));
         const uint32_t w = tree.wide[eidx];
         if (w & kLeafBit) break;
         T = w;
@@ -600,7 +601,8 @@ static int tree_create_impl(const vr_tree_desc* d, const vr_tree_quant_desc* q, 
         const int v = atoi(e);
         if (v >= 0 && v < kWideLv && max_node_depth + 1 + v <= 24) { wp = v; n_tab64 = h_pcnt[(kWideLv - v) % kWideLv] + (v ? 1 : 0); }
     }
-    if (n_tab64 * (unsigned long long)kWideEntries >= (1ull << 32)) return fail(VR_EUNSUPPORTED, "too many nodes for the wide tables");
+    // a table word holds its table's first entry index, which must stay clear of kLeafBit
+    if (n_tab64 * (unsigned long long)kWideEntries >= (1ull << 31)) return fail(VR_EUNSUPPORTED, "too many nodes for the wide tables");
     const uint32_t n_tab = (uint32_t)n_tab64;
     const long long n_entries = (long long)n_tab * kWideEntries;
     {
